@@ -2,6 +2,7 @@
 """bench.py -- env-steps/s of the b200sim CUDA path on the BASELINE.json workloads.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          our arm (one rank per GPU under torchrun for N > 1)
+  python bench.py [...] --dump-outputs DIR                     ... and what its last timed step returned, as DIR/<name>.npy
   python bench.py --impl reference [...]                       the CPU arm: this repo's fp64 restatement of the
                                                                reference's mj_step path (the reference itself cannot
                                                                be imported: `mujoco`/`gymnasium` are absent), on all
@@ -139,21 +140,20 @@ def run_reference(args, quiet=False):
         return done, time.perf_counter() - t0
 
     chunk(max(1, min(args.warmup, 3)))
-    reps = max(3, args.reps)
-    per_rep = max(1, args.steps // reps)
+    reps = min(max(3, args.reps), args.steps)
     rates = []
-    for _ in range(reps):
-        done, dt = chunk(per_rep)
+    for r in range(reps):   # args.steps env-steps in all, split as evenly as possible over the repetitions
+        done, dt = chunk(args.steps // reps + (r < args.steps % reps))
         rates.append(done / dt)
     for p, c in workers:
         c.send(0)
     for p, c in workers:
         p.join(timeout=10)
     value = statistics.median(rates)
-    sample = (f"{nenv} envs ({per} per worker process, {cores} processes) x {per_rep} env-steps per repetition, {reps} repetitions, "
+    sample = (f"{nenv} envs ({per} per worker process, {cores} processes) x {args.steps} env-steps over {reps} repetitions, "
               f"one IPC message per repetition, TimeLimit 50 + reset; liboracle built with {'-O3 -march=native' if native else '-O2'}")
     line = {"impl": "reference", "metric": "env-steps/s", "value": value, "unit": "env-steps/s", "n_gpus": args.gpus,
-            "steps": per_rep * reps, "warmup": args.warmup, "ms_per_step": 1e3 * nenv / value,
+            "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * nenv / value,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
             "config": {"workload": f"{ENV_ID}, CPU restatement of the reference mj_step path (NOT MuJoCo: dependency absent), "
                                    f"bounded sample of {nenv} envs per step", "n_substeps": 20},
@@ -249,10 +249,61 @@ def make_env(H, workload, n, rng_mode):
     return env
 
 
-def time_workload(H, workload, n, steps, warmup, rng_mode="torch", nvtx=False, sample_clocks=False, gather=False):
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def step_outputs(result):
+    """What env.step returned -- observation entries, reward, terminated, truncated and the tensors of the info dict (nested keys
+    joined with '.', info keys prefixed 'info.') -- as host arrays: float64 stays float64, integers become float64 (exact for the
+    int32 solver counters), everything else float32."""
+    import numpy as np
+    import torch
+
+    obs, reward, terminated, truncated, info = result
+    out = {}
+
+    def add(name, v):
+        if isinstance(v, dict):
+            for k, x in v.items():
+                add(f"{name}.{k}" if name else k, x)
+        elif torch.is_tensor(v):
+            a = v.detach().cpu().numpy()
+            out[name] = a.astype(np.float64 if a.dtype == np.float64 or a.dtype.kind in "iu" else np.float32)
+
+    add("" if isinstance(obs, dict) else "obs", obs)
+    add("reward", reward)
+    add("terminated", terminated)
+    add("truncated", truncated)
+    add("info", info)
+    return out
+
+
+def write_outputs(arrays, n, path):
+    """DIR/<name>.npy for every array; above DUMP_LIMIT_BYTES in all, the rows of a fixed seeded sample of the n envs (their indices
+    in env_index.npy) of every array whose first axis is the env axis."""
+    import numpy as np
+
+    budget = DUMP_LIMIT_BYTES - 1024 * (len(arrays) + 1)   # a .npy header takes at most 1 KB
+    total = sum(a.nbytes for a in arrays.values())
+    if total > budget:
+        per_env = sum(a.nbytes for a in arrays.values() if a.ndim and a.shape[0] == n) / n
+        fixed = total - per_env * n
+        keep = int((budget - fixed) // (per_env + 8))   # + 8 bytes per kept env: its float64 index
+        if keep < 1:
+            raise SystemExit(f"--dump-outputs: the outputs do not fit in {DUMP_LIMIT_BYTES} bytes")
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {k: a[idx] if a.ndim and a.shape[0] == n else a for k, a in arrays.items()}
+        arrays["env_index"] = idx.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
+def time_workload(H, workload, n, steps, warmup, rng_mode="torch", nvtx=False, sample_clocks=False, gather=False, keep_outputs=False):
     """Three timed arms over the same env: (1) `value`: CUDA events around env.step with device-resident actions, (2) the step
     kernel alone, (3) end to end with HOST buffers -- pinned actions H2D, the packed result rows D2H, every step.  All times are
-    per-rank sums; the caller takes the max over ranks."""
+    per-rank sums; the caller takes the max over ranks.  keep_outputs: res["outputs"] holds what the last step of arm (1) returned
+    (step_outputs)."""
     torch = H.torch
     env_id, nact, nsub, b_alg, _ = WORKLOADS[workload]
     env = make_env(H, workload, n, rng_mode)
@@ -276,13 +327,15 @@ def time_workload(H, workload, n, steps, warmup, rng_mode="torch", nvtx=False, s
         ev[k][0].record()
         if nv:
             nv.range_push(f"env.step {k}")
-        _, _, _, _, info = env.step(tape[k % 64])
+        last = env.step(tape[k % 64])
         if nv:
             nv.range_pop()
         ev[k][1].record()
+        info = last[4]
         if "_final_obs" in info:
             reset_masks.append(info["_final_obs"])   # same-step autoreset happened inside this timed step
     H.barrier()
+    outputs = step_outputs(last) if keep_outputs else None   # before the arms below step the env again
     ms = sum(a.elapsed_time(b) for a, b in ev)
     launches = env.backend.launches - launches0
     resets = int(sum(int(m.sum()) for m in reset_masks))
@@ -359,7 +412,7 @@ def time_workload(H, workload, n, steps, warmup, rng_mode="torch", nvtx=False, s
     res = dict(workload=workload, env_id=env_id, n=n, nsub=nsub, nact=nact, b_alg=b_alg, ms=ms, kms=kms, e2e_ms=e2e_s * 1e3,
                e2e_gather_ms=None if e2e_gather_s is None else e2e_gather_s * 1e3, launches=launches, resets=resets, h2d=h2d, d2h=d2h,
                clocks=clocks, overflow_env_steps=int(env.backend.overflow_counter[0]),
-               wpb=None, gathered_rows=None if gatherer is None else int(gatherer.rows))
+               wpb=None, gathered_rows=None if gatherer is None else int(gatherer.rows), outputs=outputs)
     env.close()
     return res
 
@@ -406,7 +459,8 @@ def run_ours(args):
         headline = mixed[rank]
         args.envs_per_gpu = args.envs_per_gpu or 1024
     n = args.envs_per_gpu or WORKLOADS[headline][4]
-    res = time_workload(H, headline, n, args.steps, args.warmup, rng_mode=args.rng_mode, nvtx=args.nvtx, sample_clocks=True, gather=args.gather)
+    res = time_workload(H, headline, n, args.steps, args.warmup, rng_mode=args.rng_mode, nvtx=args.nvtx, sample_clocks=True, gather=args.gather,
+                        keep_outputs=bool(args.dump_outputs) and rank == 0)
     if os.environ.get("B200SIM_BENCH_DEBUG"):
         print(f"[rank {rank}] ms/step {res['ms'] / args.steps:.3f} kernel {res['kms']:.3f} e2e {res['e2e_ms'] / args.steps:.3f}", file=sys.stderr)
     ms, e2e_ms, kms, e2e_g = H.max_over_ranks([res["ms"], res["e2e_ms"], res["kms"], res["e2e_gather_ms"] or 0.0])
@@ -443,6 +497,8 @@ def run_ours(args):
                             "e2e": {"value": 1024 * world * ksteps / (ce2e / 1e3), "unit": "env-steps/s", "h2d_bytes_per_step": r["h2d"],
                                     "d2h_bytes_per_step": r["d2h"]}})
     if rank == 0:
+        if args.dump_outputs:
+            write_outputs(res["outputs"], n, args.dump_outputs)
         env_id, nsub = res["env_id"], res["nsub"]
         cpu = None
         if world == 1 and not args.no_cpu_baseline and args.workload == "fetch_pick_and_place":
@@ -492,7 +548,14 @@ def main():
     ap.add_argument("--nvtx", action="store_true", help="NVTX range around every timed env.step (profiling runs only)")
     ap.add_argument("--rng-mode", default="torch", choices=["torch", "device"],
                     help="reset draws of the Fetch workload: torch's device generator (default) or in-kernel (b200sim_reset)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline workload returned as DIR/<name>.npy (rank 0's envs; "
+                         "at most 64 MB, a fixed sample of the envs above that); the inputs are seeded, so two builds can be compared")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

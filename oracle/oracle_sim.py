@@ -28,26 +28,24 @@ def use_native_build():
 
 
 def build(force: bool = False) -> str:
-    """Compile oracle.c -> oracle/_build/liboracle.so with gcc (idempotent)."""
-    name, flags = "liboracle.so", ["-O2"]
-    if _NATIVE:
-        import hashlib
-        import platform
-
-        cpu = ""
-        try:
-            cpu = next((l for l in open("/proc/cpuinfo") if l.startswith("model name")), "")
-        except OSError:
-            pass
-        name = "liboracle_native_" + hashlib.sha1((platform.machine() + cpu).encode()).hexdigest()[:10] + ".so"
-        flags = ["-O3", "-march=native"]
-    out = os.path.join(_HERE, "_build", name)
+    """Compile oracle.c -> oracle/_build/liboracle.so with gcc (idempotent).  The native build goes to a fresh temporary directory,
+    removed at exit: bench.py, its only user, runs from a tree it does not write to."""
     src = os.path.join(_HERE, "oracle.c")
+    if _NATIVE:
+        import atexit
+        import shutil
+        import tempfile
+
+        out = os.path.join(tempfile.mkdtemp(prefix="liboracle_native_"), "liboracle.so")
+        atexit.register(shutil.rmtree, os.path.dirname(out), True)
+        subprocess.check_call(["gcc", "-O3", "-march=native", "-fPIC", "-shared", "-o", out, src, "-lm"])
+        return out
+    out = os.path.join(_HERE, "_build", "liboracle.so")
     hdr = os.path.join(_HERE, "..", "include", "b200sim_model.h")
     if force or not os.path.exists(out) or (os.path.exists(src) and os.path.getmtime(out) < max(os.path.getmtime(src), os.path.getmtime(hdr))):
         os.makedirs(os.path.dirname(out), exist_ok=True)
         tmp = f"{out}.{os.getpid()}.tmp"
-        subprocess.check_call(["gcc"] + flags + ["-fPIC", "-shared", "-o", tmp, src, "-lm"])
+        subprocess.check_call(["gcc", "-O2", "-fPIC", "-shared", "-o", tmp, src, "-lm"])
         os.replace(tmp, out)
     return out
 

@@ -7,12 +7,9 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-REFERENCE_ASSETS = "/root/reference/gymnasium_robotics/envs/assets"
-
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "needs_reference: needs /root/reference (build container only)")
 
 
 def pytest_collection_modifyitems(config, items):
@@ -22,8 +19,6 @@ def pytest_collection_modifyitems(config, items):
     for item in items:
         if "gpu" in item.keywords and not has_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
-        if "needs_reference" in item.keywords and not os.path.isdir(REFERENCE_ASSETS):
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present"))
 
 
 @pytest.fixture

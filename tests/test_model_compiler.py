@@ -1,11 +1,19 @@
-"""MJCF -> constant tables: sizes, MuJoCo compile rules, blob round trip, committed blobs in sync with the sources."""
+"""MJCF -> constant tables: sizes, MuJoCo compile rules, blob round trip, committed blobs in sync with the sources.
+
+The reference's MJCF assets are not redistributed: what the tests below need from them (digests of a fresh compile, masses and an
+inertial frame read from fetch/robot.xml, the unfused mass matrix) is recorded in golden/fetch_model_facts.json by
+golden/make_fetch_model_facts.py."""
+import hashlib
+import json
 import os
 
 import numpy as np
 import pytest
 
 from gymnasium_robotics_b200.mjcf import Model, compile_mjcf
-from gymnasium_robotics_b200.models import MODEL_DIR, MODEL_OVERRIDES, MODEL_SOURCES, REFERENCE_ASSETS, load_model
+from gymnasium_robotics_b200.models import MODEL_DIR, MODEL_SOURCES, load_model
+
+FACTS = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "fetch_model_facts.json")))
 
 
 def test_committed_blobs_load_and_have_expected_sizes():
@@ -25,23 +33,22 @@ def test_blob_round_trip_is_lossless():
     assert m.names == m2.names
 
 
-@pytest.mark.needs_reference
 def test_committed_blobs_match_a_fresh_compile():
-    for name, rel in MODEL_SOURCES.items():
-        fresh = compile_mjcf(os.path.join(REFERENCE_ASSETS, rel), overrides=MODEL_OVERRIDES.get(name)).to_blob()
-        assert open(os.path.join(MODEL_DIR, name + ".b200m"), "rb").read() == fresh, name
+    assert sorted(FACTS["blob_sha256"]) == sorted(MODEL_SOURCES)
+    for name, digest in FACTS["blob_sha256"].items():
+        assert hashlib.sha256(open(os.path.join(MODEL_DIR, name + ".b200m"), "rb").read()).hexdigest() == digest, name
 
 
-@pytest.mark.needs_reference
 def test_fused_runtime_model_keeps_the_dynamics():
     """Fusing jointless bodies (MuJoCo `fusestatic`) must not change the mass matrix; collision filters follow MuJoCo."""
     from oracle.oracle_sim import OracleSim
 
-    m = compile_mjcf(os.path.join(REFERENCE_ASSETS, "fetch/pick_and_place.xml"))
+    m = load_model("fetch_pick_and_place")
+    full = FACTS["fetch_pick_and_place_mjcf"]
     s = OracleSim(m)
     s.forward()
-    assert np.abs(s.M - m._full_arrays["M0"]).max() < 1e-10  # oracle CRB on the fused tree vs dense sum on the MJCF tree
-    assert m.nbody == 16 and len(m._full.bodies) == 33  # 33 MJCF bodies (world included) fuse into 16
+    assert np.abs(s.M - np.array(full["M0"])).max() < 1e-10  # oracle CRB on the fused tree vs dense sum on the MJCF tree
+    assert m.nbody == 16 and full["bodies"] == 33  # 33 MJCF bodies (world included) fuse into 16
     geoms = m.names["geom"]
     pairs = {(geoms[a], geoms[b]) for a, b in zip(m.pair_geom1, m.pair_geom2)}
     assert ("robot0:r_gripper_finger_link", "robot0:l_gripper_finger_link") not in pairs  # <exclude>
@@ -74,28 +81,6 @@ def test_defaults_childclass_euler_fromto(mjcf_file):
 # error in the compiler (inertia from geoms / <inertial>, fusing, invweight0) is common-mode and invisible to the parity tests;
 # these tests anchor the constants to numbers taken straight from the XML text and to a second computation path (the C oracle's
 # kinematics + mass matrix, finite-difference Jacobians, numpy), not to the compiler's own arithmetic.
-def _xml_subtree_masses(path):
-    """{body name: sum of the <inertial mass=...> entries of the body's subtree}, read from the MJCF text with ElementTree
-    (fetch/robot.xml gives every link an explicit <inertial>; geoms of such bodies do not add mass)."""
-    import xml.etree.ElementTree as ET
-
-    out = {}
-
-    def walk(b):
-        tot = sum(float(i.get("mass")) for i in b.findall("inertial"))
-        for ch in b.findall("body"):
-            tot += walk(ch)
-        out[b.get("name")] = tot
-        return tot
-
-    root = ET.parse(path).getroot()
-    for b in root.iter("body"):
-        if b.get("name") not in out:
-            walk(b)
-    return out
-
-
-@pytest.mark.needs_reference
 def test_fetch_closed_form_totals():
     """Total robot mass, the composite inertia seen by the three base slides, and the gravity load on the torso lift joint of the
     Fetch model: XML numbers against the compiled blob, the oracle (C, fp64) and the kernel emulation (fp32)."""
@@ -103,7 +88,7 @@ def test_fetch_closed_form_totals():
     from tests.hostsim import HostSim
     from gymnasium_robotics_b200.fetch import REF_POINT, welded_eq_data
 
-    sub = _xml_subtree_masses(os.path.join(REFERENCE_ASSETS, "fetch", "robot.xml"))
+    sub = FACTS["fetch_robot_xml"]["subtree_mass"]
     robot_mass = sub["robot0:base_link"]
     assert robot_mass == pytest.approx(70.1294 + 10.7796 + 2.2556 + 0.9087 + 2.5587 + 2.6615 + 2.3311 + 2.1299 + 1.6563 + 1.725 + 0.1354 + 1.5175 +
                                        4 + 4 + 0.002 + 0.0083 + 13.2775, abs=1e-9)
@@ -133,13 +118,10 @@ def test_fetch_closed_form_totals():
     assert hs.fsmooth[d] == pytest.approx(passive_and_act - load, rel=5e-6)
 
 
-@pytest.mark.needs_reference
 def test_invweight0_recomputed_along_a_second_path():
     """dof_invweight0 = diag(M^-1) and the weld's body_invweight0 = block averages of J M^-1 J^T at qpos0 -- recomputed from the C
     oracle's mass matrix and finite-difference Jacobians of its kinematics (the compiler uses analytic Jacobians on the unfused
     tree in numpy), plus the free box whose values are closed-form (1/m and the mean of 1/I)."""
-    import xml.etree.ElementTree as ET
-
     from oracle.oracle_sim import OracleSim
 
     m = load_model("fetch_pick_and_place")
@@ -150,8 +132,7 @@ def test_invweight0_recomputed_along_a_second_path():
     assert np.allclose(np.diag(Minv), m.dof_invweight0, rtol=1e-9)
     # weld robot0:mocap <-> robot0:gripper_link: invweight = that of the gripper link (the mocap body has no dofs)
     site = m.frame_site("robot0:gripper_link")
-    g = next(b for b in ET.parse(os.path.join(REFERENCE_ASSETS, "fetch", "robot.xml")).getroot().iter("body") if b.get("name") == "robot0:gripper_link")
-    ipos = np.array([float(x) for x in g.find("inertial").get("pos").split()])
+    ipos = np.array(FACTS["fetch_robot_xml"]["gripper_link_inertial_pos"])
 
     def com():
         return s.site_xpos[site] + s.site_xmat[site].reshape(3, 3) @ ipos
