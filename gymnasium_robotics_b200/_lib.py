@@ -127,11 +127,12 @@ def lib():
     L.b200sim_launch_count.argtypes = [vp]
     L.b200sim_launch_count.restype = ctypes.c_long
     L.b200sim_launch_config.argtypes = [vp, ctypes.POINTER(ci), ctypes.POINTER(ci), ctypes.POINTER(ci)]
+    L.b200sim_kernel_variant.argtypes = [vp, ctypes.POINTER(ci), ctypes.POINTER(ci), ctypes.POINTER(ci)]
     _LIB = L
     return L
 
 
 EXPORTED_SYMBOLS = ["b200sim_create", "b200sim_destroy", "b200sim_last_error", "b200sim_num_envs", "b200sim_layout",
                     "b200sim_state", "b200sim_step", "b200sim_refresh", "b200sim_raw_step", "b200sim_raw_step_masked", "b200sim_compute_reward", "b200sim_reset", "b200sim_reset_uniform", "b200sim_reset_maze", "b200sim_check_state", "b200sim_reset_reach", "b200sim_reset_hand_pose", "b200sim_reset_hand_goal",
-                    "b200sim_launch_count", "b200sim_launch_config", "b200sim_set_time_limit", "b200sim_elapsed", "b200sim_overflow_counter",
+                    "b200sim_launch_count", "b200sim_launch_config", "b200sim_kernel_variant", "b200sim_set_time_limit", "b200sim_elapsed", "b200sim_overflow_counter",
                     "b200sim_packed_width", "b200sim_set_packed"]

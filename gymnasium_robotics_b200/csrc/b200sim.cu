@@ -372,6 +372,13 @@ int b200sim_launch_config(const b200sim_t* h, int* smem_bytes, int* envs_per_blo
   if (blocks) *blocks = h->blocks;
   return 0;
 }
+int b200sim_kernel_variant(const b200sim_t* h, int* envs_per_block, int* nvp, int* build) {
+  if (envs_per_block) *envs_per_block = h->wpb;
+  if (nvp) *nvp = h->nvp;
+  if (build) *build = h->hull ? B200SIM_BUILD_KITCHEN_HULL : (h->kitchen ? (h->kitchen_groups ? B200SIM_BUILD_KITCHEN_GROUPS : B200SIM_BUILD_KITCHEN_FLAT)
+                                                                   : (h->nvp == B200_WIDE_NVP ? B200SIM_BUILD_WIDE : B200SIM_BUILD_ARM));
+  return 0;
+}
 int b200sim_set_time_limit(b200sim_t* h, int max_episode_steps, int terminate_on_success) {
   h->max_steps = max_episode_steps > 0 ? max_episode_steps : 0;
   h->term_on_success = terminate_on_success ? 1 : 0;

@@ -195,6 +195,14 @@ int b200sim_compute_reward(const b200sim_t* h, const float* achieved, const floa
 long b200sim_launch_count(const b200sim_t* h);
 /* shared-memory bytes per block and warps (envs) per block chosen at create time */
 int b200sim_launch_config(const b200sim_t* h, int* smem_bytes, int* envs_per_block, int* blocks);
+/* which step-kernel instantiation this handle launches: envs per block, the padded dof count NVP of the template, and the build
+ * (translation unit) it lives in.  Read-only; any pointer may be NULL. */
+enum { B200SIM_BUILD_ARM = 0,            /* b200sim.cu: Fetch, mazes, Shadow Hand, Adroit up to 30 dofs */
+       B200SIM_BUILD_WIDE = 1,           /* b200sim_wide.cu: 33..36 dofs */
+       B200SIM_BUILD_KITCHEN_FLAT = 2,   /* b200sim_kitchen.cu (B200SIM_KITCHEN_GROUPS=0) */
+       B200SIM_BUILD_KITCHEN_GROUPS = 3, /* b200sim_kitchen_groups.cu */
+       B200SIM_BUILD_KITCHEN_HULL = 4 }; /* b200sim_kitchen_hull.cu */
+int b200sim_kernel_variant(const b200sim_t* h, int* envs_per_block, int* nvp, int* build);
 
 #ifdef __cplusplus
 }
